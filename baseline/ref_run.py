@@ -6,7 +6,7 @@ container has no `plyfile`, and BASELINE.md §3.1 excludes file parsing from the
     load_transform_data(path, skip_rate)  -> ({name: 4x4 nested list}, {name: [w, h, fx, fy]})
 
   run(scene, cams, intr, settings_kwargs, device)   device "cuda:0": stock GPU path (renderer_type "cuda" uses the
-                                                     reference's CUDA rasterizer built by baseline/build_ref.py)
+                                                     reference's CUDA rasterizer built by oracle/build_ref.py)
                                                      device "cpu": through oracle.ref_shim.cpu_redirect (the
                                                      reference hard-codes "cuda" devices)
 Used by bench.py's reference legs and by GPU tests that compare against the reference itself.  Never imported by the

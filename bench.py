@@ -18,7 +18,7 @@ c4 = c3's scene, 50M points, surface_distance_std 2.0, exact_num_points (rendere
 Extra objects in the JSON line (all measured in this run, on this box):
   roofline        the dominant kernel of the step (by summed CUDA-event time) against the roof that bounds it
   rooflines       every hand-written kernel: algorithmic bytes / event time vs the measured HBM peak
-  ref_cuda        the UNMODIFIED reference pipeline with its CUDA rasterizer (baseline/_ref, built for sm_100) on the same
+  ref_cuda        the UNMODIFIED reference pipeline with its CUDA rasterizer (oracle/_ref, built for sm_100) on the same
                   workload and GPU — the ">= 10x" comparator of BASELINE.md §3.5
   c1              config C1 like for like: this build (GPU) next to the reference's own code on the host cores, in full
   cpu_baseline    the reference's own python path on a bounded sample of the workload (host cores)
@@ -70,7 +70,31 @@ def parse():
     ap.add_argument("--no-c1", action="store_true")
     ap.add_argument("--cpu-sample-gaussians", type=int, default=30000)
     ap.add_argument("--cpu-sample-cams", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the point cloud of the last timed step to DIR/<name>.npy (a fixed row sample if large)")
     return ap.parse_args()
+
+
+DUMP_MAX_ROWS = 700_000  # rows kept per array: 3 arrays x 700 k rows x 3 x 8 B = 50.4 MB even if all are float64
+
+
+def dump_outputs(pc, out_dir, suffix=""):
+    """points / colours / normals of a PointCloudData as float32 (float64 kept) .npy files; more than DUMP_MAX_ROWS rows
+    are reduced to the same seeded, sorted row sample in every array, so two builds that agree on the cloud agree here."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = int(pc.points.shape[0])
+    rows = None
+    if n > DUMP_MAX_ROWS:
+        g = torch.Generator().manual_seed(0)
+        rows = torch.randperm(n, generator=g)[:DUMP_MAX_ROWS].sort().values
+    for name in ("points", "colours", "normals"):
+        t = getattr(pc, name)
+        if t is None:
+            continue
+        if rows is not None:
+            t = t[rows.to(t.device)]
+        a = t.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a if a.dtype == np.float64 else a.astype(np.float32))
 
 
 def settings_for(wl, g2p, device, renderer=None):
@@ -282,6 +306,8 @@ def run_ours(args):
         ms, npts, pc = timed(step_resident, args.steps)
         clk.mark_end()
     launches = capi.LAUNCHES
+    if args.dump_outputs:
+        dump_outputs(pc, args.dump_outputs, f"_rank{rank}" if world > 1 else "")
     ms_step = ms / args.steps
     value = npts / (ms_step * 1e-3) / 1e6
 
@@ -441,7 +467,7 @@ def ref_cuda_leg(wl, our_e2e):
         from baseline import ref_run
         from g2pc import synth
         if not (ref_run.available() and ref_run.cuda_extension_available()):
-            return {"unavailable": "baseline/_ref not staged (run baseline/build_ref.py in the build container)"}
+            return {"unavailable": "reference not available (G2PC_REFERENCE_ROOT unset or oracle/build_ref.py not run)"}
         sc = _scene_for(wl)
         cams, intr = synth.make_cameras(wl["cams"])
         kw = dict(renderer_type="cuda", num_points=wl["points"], colour_resolution=wl["res"], max_sh_degree=wl["sh"],
@@ -507,7 +533,7 @@ def c1_leg(g2p, capi, sampler, dev):
 
 
 def reference_c1(steps=5):
-    """The reference's OWN code (unmodified, staged under baseline/_ref/py or /root/reference) on C1 in full, CPU."""
+    """The reference's OWN code (unmodified, the checkout named by $G2PC_REFERENCE_ROOT) on C1 in full, CPU."""
     try:
         from baseline import ref_run
         if not ref_run.available():

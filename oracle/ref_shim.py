@@ -1,7 +1,7 @@
-"""Run the UNMODIFIED reference (/root/reference) on CPU in the build container (TEST INFRASTRUCTURE).
+"""Run the UNMODIFIED reference (the checkout named by $G2PC_REFERENCE_ROOT) on CPU (TEST INFRASTRUCTURE).
 
-Used only by tests/golden/make_golden.py to produce the committed golden vectors that pin the oracle, and by
-`-m "not gpu"` tests that are skipped when /root/reference is absent (it does not exist on the GPU box).
+Used by tests/golden/make_golden.py to produce the committed golden vectors that pin the oracle, and by bench.py's
+reference legs; the tests compare against those vectors and never need the reference itself.
 
 What the shim does (no reference source is edited or copied):
   * stubs the three import-time modules the container lacks (configargparse, imageio, plyfile);
@@ -22,27 +22,16 @@ import numpy as np
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# staged byte-for-byte copy of the reference's Python modules (baseline/build_ref.py; git-ignored, travels to the GPU box)
-STAGED_ROOT = os.path.join(os.path.dirname(_HERE), "baseline", "_ref", "py")
-STAGED_EXT_ROOT = os.path.join(os.path.dirname(_HERE), "baseline", "_ref")
-
-
-def _find_root():
-    env = os.environ.get("G2PC_REFERENCE_ROOT")
-    for cand in ([env] if env else []) + ["/root/reference", STAGED_ROOT]:
-        if cand and os.path.isfile(os.path.join(cand, "gauss_to_pc.py")):
-            return cand
-    return env or "/root/reference"
-
-
-REF_ROOT = _find_root()
+# the reference's compiled CUDA extension (oracle/build_ref.py; git-ignored)
+STAGED_EXT_ROOT = os.path.join(_HERE, "_ref")
+REF_ROOT = os.environ.get("G2PC_REFERENCE_ROOT", "")
 
 _FACTORIES = ["zeros", "ones", "full", "eye", "tensor", "arange", "empty", "zeros_like", "ones_like", "full_like",
               "empty_like", "linspace", "rand", "randn", "as_tensor"]
 
 
 def available():
-    return os.path.isfile(os.path.join(REF_ROOT, "gauss_to_pc.py"))
+    return bool(REF_ROOT) and os.path.isfile(os.path.join(REF_ROOT, "gauss_to_pc.py"))
 
 
 def _is_cuda_dev(d):
@@ -119,21 +108,22 @@ _ref_ext = None
 
 
 def _load_reference_extension():
-    """The reference's OWN package `gaussian_pointcloud_rasterization` (wrapper + _C built by baseline/build_ref.py),
-    imported from baseline/_ref under a private module object — the product ships a package of the same name."""
+    """The reference's OWN package `gaussian_pointcloud_rasterization` (its wrapper from REF_ROOT, _C built by
+    oracle/build_ref.py), imported under a private module object — the product ships a package of the same name."""
     global _ref_ext
     if _ref_ext is not None:
         return _ref_ext
     import importlib.util
+    src_dir = os.path.join(REF_ROOT, "gaussian-pointcloud-rasterization", "gaussian_pointcloud_rasterization")
     pkg_dir = os.path.join(STAGED_EXT_ROOT, "gaussian_pointcloud_rasterization")
-    init = os.path.join(pkg_dir, "__init__.py")
-    if not os.path.isfile(init):
+    init = os.path.join(src_dir, "__init__.py")
+    if not (os.path.isfile(init) and os.path.isdir(pkg_dir)):
         return None
     saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "gaussian_pointcloud_rasterization"
              or k.startswith("gaussian_pointcloud_rasterization.")}
     try:
         spec = importlib.util.spec_from_file_location("gaussian_pointcloud_rasterization", init,
-                                                      submodule_search_locations=[pkg_dir])
+                                                      submodule_search_locations=[src_dir, pkg_dir])
         mod = importlib.util.module_from_spec(spec)
         sys.modules["gaussian_pointcloud_rasterization"] = mod
         spec.loader.exec_module(mod)  # imports ._C from pkg_dir
@@ -153,7 +143,7 @@ def reference_extension():
     camera_handler.py:73) resolves to the REFERENCE's package, not the product's."""
     ext = _load_reference_extension()
     if ext is None:
-        raise RuntimeError("reference CUDA extension not staged (baseline/build_ref.py)")
+        raise RuntimeError("reference CUDA extension not built (oracle/build_ref.py)")
     names = [k for k in sys.modules if k == "gaussian_pointcloud_rasterization"
              or k.startswith("gaussian_pointcloud_rasterization.")]
     saved = {k: sys.modules.pop(k) for k in names}
@@ -175,7 +165,7 @@ def load():
     if _loaded is not None:
         return _loaded
     if not available():
-        raise RuntimeError(f"reference not found under {REF_ROOT}")
+        raise RuntimeError("reference not found: set G2PC_REFERENCE_ROOT to its checkout")
     _stub_modules()
     # the reference modules are top-level scripts; import them under their own names from REF_ROOT only
     names = ["gauss_handler", "gauss_render", "camera_handler", "gauss_dataloader", "transform_dataloader",

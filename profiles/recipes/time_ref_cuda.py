@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Time the UNMODIFIED reference pipeline with renderer_type=cuda (the reference CUDA rasterizer built for sm_100 by
-baseline/build_ref.py) on a bench.py workload, with a colour-stage / sampling-stage split.
+oracle/build_ref.py) on a bench.py workload, with a colour-stage / sampling-stage split.
 
     python profiles/recipes/time_ref_cuda.py --workload c3 --steps 1 [--json out.json]
 """

@@ -1,11 +1,14 @@
-"""Generate the golden vectors that pin the oracle: outputs of the UNMODIFIED reference (/root/reference) run on
-CPU through oracle/ref_shim.py on small seeded scenes.  Run in the build container (the reference does not exist on
-the GPU box):
+"""Generate the golden vectors that pin the oracle and the kernels: outputs of the UNMODIFIED reference on small
+seeded scenes.  The CPU cases run the reference's Python code through oracle/ref_shim.py:
 
-    python tests/golden/make_golden.py
+    G2PC_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py [case ...]
 
-Writes tests/golden/sampling_*.npz (and colour_*.npz).  Inputs are regenerated from the seeds by g2pc.synth, so only
-outputs are stored.
+The `ref_ext` case runs the reference's compiled CUDA rasterizer (oracle/build_ref.py) on a GPU and needs no other
+part of the reference:
+
+    python tests/golden/make_golden.py ref_ext [output directory]
+
+Inputs are regenerated from the seeds by g2pc.synth (and the test helpers), so only outputs are stored.
 """
 import os
 import sys
@@ -97,10 +100,121 @@ def make_sh(name="sh_a", n=400, seed=1320):
     print(name, {k: v.shape for k, v in out.items()})
 
 
+def make_live_small(name="live_small", n=600, scene_seed=77, num_points=5000, rng_seed=5):
+    """generate_pointcloud of the reference (gauss_to_pc.py:73-371) with the product's eps, default arguments."""
+    ref = ref_shim.load()
+    sc = synth.make_scene(n, seed=scene_seed)
+    eps_fn = lambda g, k, a: philox.draw_eps(g, k, a, rng_seed, 0)
+    with ref_shim.cpu_redirect():
+        G = ref.gauss_handler.Gaussians(sc["xyz"].clone(), sc["scales"].clone(), sc["rots"].clone(),
+                                        sc["colours"].clone() * 255, sc["opacities"].clone())
+        G.calculate_normals()
+        G.validate_covariances()
+        with ref_shim.EpsInjector(ref, G.xyz, eps_fn):
+            pts, cols, nrm = ref.gauss_to_pc.generate_pointcloud(G, num_points, device="cpu", quiet=True)
+    np.savez_compressed(os.path.join(HERE, name + ".npz"),
+                        meta=np.array([n, scene_seed, num_points, rng_seed], dtype=np.int64),
+                        points=pts.numpy(), colours=cols.numpy())
+    print(name, "points", tuple(pts.shape), pts.dtype, cols.dtype)
+
+
+TRANSFORM_KINDS = ("json", "colmap_txt", "colmap_bin")
+
+
+def make_transforms(name="transforms"):
+    """load_transform_data of the reference (transform_dataloader.py) on the files tests/test_io_cpu.py writes."""
+    import tempfile
+    sys.path.insert(0, os.path.dirname(HERE))
+    import test_io_cpu as tio
+    ref = ref_shim.load()
+    out = {}
+    with tempfile.TemporaryDirectory() as tmp:
+        for kind in TRANSFORM_KINDS:
+            path = tio.write_transform_files(tmp, kind)
+            for skip in (0, 2):
+                tr, ik = ref.transform_dataloader.load_transform_data(path, skip_rate=skip)
+                out[f"{kind}_skip{skip}_names"] = np.array(list(tr.keys()))
+                out[f"{kind}_skip{skip}_c2w"] = np.array([np.asarray(tr[k], dtype=np.float64) for k in tr])
+                out[f"{kind}_skip{skip}_intrinsics"] = np.array([[float(v) for v in ik[k]] for k in tr])
+    np.savez_compressed(os.path.join(HERE, name + ".npz"), **out)
+    print(name, {k: v.shape for k, v in out.items()})
+
+
+# n_gaussians, scene_seed, n_cameras, colour_resolution, sampled pixels per image, pixel-sample seed
+REF_EXT_CASE = (20000, 1253, 4, 720, 12000, 7)
+
+
+def load_reference_extension():
+    """The reference's compiled `_C` module (oracle/build_ref.py) under a private name; its Python wrapper is not
+    needed: the op's 22 arguments are assembled here exactly as the wrapper does (GaussianRasterizer.forward)."""
+    import importlib.util
+    from oracle import build_ref
+    path = build_ref.extension_path()
+    if path is None:
+        raise SystemExit("reference extension not built: run oracle/build_ref.py")
+    spec = importlib.util.spec_from_file_location("g2pc_reference_ext._C", path)
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
+def make_ref_ext(out_dir, name="ref_ext_a"):
+    """The reference CUDA rasterizer (renderer_type "cuda", colours precomputed, surface distance on) on REF_EXT_CASE:
+    per camera the radii and a fixed pixel sample of the image and depth; per Gaussian the maximum / total
+    contribution and the minimum surface distance accumulated over the cameras as the reference's wrapper does."""
+    import camera_handler as ch
+    from oracle import gaussians as og
+    _C = load_reference_extension()
+    n, scene_seed, ncams, res, n_pix, pix_seed = REF_EXT_CASE
+    dev = "cuda:0"
+    sc = synth.make_scene(n, seed=scene_seed, sh_degree=3)
+    cov = og.build_covariance(sc["scales"], sc["rots"])
+    xyz, opac = sc["xyz"].to(dev).float(), sc["opacities"].to(dev).unsqueeze(1).float()
+    colours = sc["colours"].to(dev).float()
+    cov6 = cov.to(dev).reshape(-1, 9)[:, [0, 1, 2, 4, 5, 8]].float()  # strip_symmetric
+    empty = torch.Tensor([])
+    max_c = torch.zeros(n, device=dev)
+    tot_c = torch.zeros(n, device=dev)
+    min_sd = torch.full((n,), torch.finfo(torch.float).max, device=dev)
+    cams, intr = synth.make_cameras(ncams)
+    radii_all, img_s, dep_s, pix = [], [], [], None
+    for c2w, k in zip(cams, intr):
+        rs = ch.get_camera("cuda", c2w.to(dev), k, colour_resolution=res)
+        H, W = rs.image_height, rs.image_width
+        if pix is None:
+            pix = np.sort(np.random.default_rng(pix_seed).choice(H * W, n_pix, replace=False)).astype(np.int32)
+        mask = torch.full((H * W,), 1, device=dev, dtype=torch.int)
+        out = _C.rasterize_gaussians(rs.bg, xyz, colours, opac, empty, empty, rs.scale_modifier, cov6, rs.viewmatrix,
+                                     rs.projmatrix, rs.tanfovx, rs.tanfovy, H, W, empty, rs.sh_degree, rs.campos, mask,
+                                     rs.prefiltered, rs.antialiasing, True, rs.debug)
+        _, colour, depth, radii, _, _, _, _, contrib, surf, _ = out
+        upd = contrib > max_c
+        max_c[upd] = contrib[upd]
+        tot_c += contrib
+        upd = surf < min_sd
+        min_sd[upd] = surf[upd]
+        assert int(radii.max()) < 2 ** 15
+        radii_all.append(radii.cpu().numpy().astype(np.int16))
+        img_s.append(colour.reshape(3, -1)[:, pix].cpu().numpy())
+        dep_s.append(depth.reshape(-1)[pix].cpu().numpy())
+    path = os.path.join(out_dir, name + ".npz")
+    np.savez_compressed(path, meta=np.array(REF_EXT_CASE, dtype=np.int64), image_hw=np.array([H, W]), pixels=pix,
+                        radii=np.stack(radii_all), image=np.stack(img_s), depth=np.stack(dep_s),
+                        max_contribution=max_c.cpu().numpy(), total_contribution=tot_c.cpu().numpy(),
+                        min_surface_distance=min_sd.cpu().numpy())
+    print(name, path, os.path.getsize(path), "bytes")
+
+
+CPU_CASES = {"sh": make_sh,
+             **{k: (lambda k=k: make_sampling(k, *SAMPLING_CASES[k])) for k in SAMPLING_CASES},
+             **{k: (lambda k=k: make_colour(k, *COLOUR_CASES[k])) for k in COLOUR_CASES},
+             "live_small": make_live_small, "transforms": make_transforms}
+
+
 if __name__ == "__main__":
     torch.manual_seed(0)
-    make_sh()
-    for name, args in SAMPLING_CASES.items():
-        make_sampling(name, *args)
-    for name, args in COLOUR_CASES.items():
-        make_colour(name, *args)
+    if sys.argv[1:2] == ["ref_ext"]:
+        make_ref_ext(sys.argv[2] if len(sys.argv) > 2 else HERE)
+    else:
+        for case in sys.argv[1:] or list(CPU_CASES):
+            CPU_CASES[case]()

@@ -1,5 +1,6 @@
-"""CPU: the thin host-side loaders (3dgs-to-pc_b200/gauss_dataloader.py, transform_dataloader.py) — self-consistency and,
-when /root/reference is present, equality with the reference's own parsers on generated COLMAP / transforms.json files."""
+"""CPU: the thin host-side loaders (3dgs-to-pc_b200/gauss_dataloader.py, transform_dataloader.py) — self-consistency and
+equality with the reference's own parsers on generated COLMAP / transforms.json files (their outputs are stored in
+tests/golden/transforms.npz by tests/golden/make_golden.py)."""
 import json
 import os
 import struct
@@ -104,30 +105,38 @@ def _write_colmap(dirpath, cams_c2w, binary):
                 f.write("1.0 2.0 -1 3.0 4.0 -1\n")
 
 
+def write_transform_files(dirpath, kind):
+    """The camera file(s) of one loader kind for 7 synthetic cameras; returns the path to load."""
+    from g2pc import synth
+    cams, intr = synth.make_cameras(7)
+    if kind == "json":
+        path = os.path.join(dirpath, "transforms.json")
+        write_transforms_json(path, cams, intr)
+    else:
+        path = os.path.join(dirpath, kind)
+        _write_colmap(path, cams, binary=(kind == "colmap_bin"))
+    return path
+
+
 @pytest.mark.parametrize("kind", ["json", "colmap_txt", "colmap_bin"])
 def test_transform_loaders_match_reference(tmp_path, kind):
     import transform_dataloader as td
     from g2pc import synth
+    from util import GOLDEN
     cams, intr = synth.make_cameras(7)
-    if kind == "json":
-        path = str(tmp_path / "transforms.json")
-        write_transforms_json(path, cams, intr)
-    else:
-        path = str(tmp_path / kind)
-        _write_colmap(path, cams, binary=(kind == "colmap_bin"))
+    path = write_transform_files(str(tmp_path), kind)
+    g = np.load(os.path.join(GOLDEN, "transforms.npz"))
     for skip in (0, 2):
         tr, ik = td.load_transform_data(path, skip_rate=skip)
         assert len(tr) >= 1 and set(tr.keys()) <= set(ik.keys())
         for k, m in tr.items():
             assert np.asarray(m).shape == (4, 4)
-        from oracle import ref_shim
-        if ref_shim.available():
-            ref = ref_shim.load()
-            rtr, rik = ref.transform_dataloader.load_transform_data(path, skip_rate=skip)
-            assert list(rtr.keys()) == list(tr.keys())
-            for k in tr:
-                assert np.allclose(np.asarray(tr[k], dtype=np.float64), np.asarray(rtr[k], dtype=np.float64), atol=1e-12)
-                assert [float(v) for v in ik[k]] == [float(v) for v in rik[k]]
+        rnames = [str(v) for v in g[f"{kind}_skip{skip}_names"]]
+        rc2w, rik = g[f"{kind}_skip{skip}_c2w"], g[f"{kind}_skip{skip}_intrinsics"]
+        assert list(tr.keys()) == rnames
+        for i, k in enumerate(tr):
+            assert np.allclose(np.asarray(tr[k], dtype=np.float64), rc2w[i], atol=1e-12)
+            assert [float(v) for v in ik[k]] == [float(v) for v in rik[i]]
     if kind == "json":
         tr, ik = td.load_transform_data(path)
         assert np.allclose(np.asarray(tr["frame_0003"]), cams[3].numpy())

@@ -1,5 +1,5 @@
 """CPU: the oracle restatement against the committed golden vectors (outputs of the unmodified reference, generated
-by tests/golden/make_golden.py) and — when /root/reference is present — against the live reference."""
+by tests/golden/make_golden.py)."""
 import os
 
 import numpy as np
@@ -78,8 +78,8 @@ def _sh_inputs(n, seed):
 
 def test_sh_colour_matches_reference_eval_sh():
     """oracle.render.sh_colour == clamp(eval_sh + 0.5, 0) of the reference (gauss_render.py:43-99), degrees 0-3:
-    against the committed golden (outputs of the unmodified eval_sh) and, in the build container, the live function."""
-    from oracle import ref_shim, render as orr
+    against the committed golden (outputs of the unmodified eval_sh)."""
+    from oracle import render as orr
     g = np.load(os.path.join(GOLDEN, "sh_a.npz"))
     n, seed = [int(v) for v in g["meta"]]
     sh, d = _sh_inputs(n, seed)
@@ -87,9 +87,6 @@ def test_sh_colour_matches_reference_eval_sh():
         want = np.maximum(g[f"deg{deg}"] + np.float32(0.5), 0)
         got = orr.sh_colour(deg, sh[..., : (deg + 1) ** 2], d).numpy()
         assert np.abs(got - want).max() <= 2.4e-7, f"deg {deg}"  # same polynomial, fp32 association only
-        if ref_shim.available():
-            live = ref_shim.load().gauss_render.eval_sh(deg, sh[..., : (deg + 1) ** 2], d).numpy()
-            assert np.array_equal(live, g[f"deg{deg}"]), "golden is stale"
 
 
 def test_philox_known_answers():
@@ -117,24 +114,16 @@ def test_eps_stream_statistics():
 
 
 def test_live_reference_matches_oracle_small():
-    """Runs the unmodified reference through the shim (build container only)."""
-    from oracle import ref_shim
-    if not ref_shim.available():
-        pytest.skip("/root/reference not present (GPU box)")
+    """The oracle's generate_pointcloud with default arguments against the unmodified reference's (stored by
+    tests/golden/make_golden.py: live_small), both drawing the same eps."""
     from g2pc import synth
     from oracle import gaussians as og, philox, sampling as osamp
-    ref = ref_shim.load()
-    sc = synth.make_scene(600, seed=77)
-    eps_fn = lambda g, k, a: philox.draw_eps(g, k, a, 5, 0)
-    with ref_shim.cpu_redirect():
-        G = ref.gauss_handler.Gaussians(sc["xyz"].clone(), sc["scales"].clone(), sc["rots"].clone(),
-                                        sc["colours"].clone() * 255, sc["opacities"].clone())
-        G.calculate_normals()
-        G.validate_covariances()
-        with ref_shim.EpsInjector(ref, G.xyz, eps_fn):
-            pts, cols, nrm = ref.gauss_to_pc.generate_pointcloud(G, 5000, device="cpu", quiet=True)
+    g = _load("live_small")
+    n, scene_seed, num_points, rng_seed = [int(v) for v in g["meta"]]
+    sc = synth.make_scene(n, seed=scene_seed)
+    eps_fn = lambda gid, k, a: philox.draw_eps(gid, k, a, rng_seed, 0)
     cov, _ = og.validate_covariances(og.build_covariance(sc["scales"], sc["rots"]))
     nr = og.calculate_normals(sc["scales"], sc["rots"])
     o = osamp.generate_pointcloud(sc["xyz"], cov, sc["colours"] * 255, nr, og.gaussian_magnitudes(cov, sc["opacities"]),
-                                  5000, eps_fn=eps_fn)
-    assert torch.equal(o["points"], pts) and torch.equal(o["colours"], cols)
+                                  num_points, eps_fn=eps_fn)
+    assert torch.equal(o["points"], torch.from_numpy(g["points"])) and torch.equal(o["colours"], torch.from_numpy(g["colours"]))

@@ -1,6 +1,6 @@
 """GPU parity tests of the renderer_type="cuda" colour back-end (csrc/s7_tiles.cu through the C ABI):
   * against the CPU oracle oracle/render_cuda.py (restatement of the reference's CUDA rasterizer, deterministic);
-  * against the UNMODIFIED reference extension itself on the GPU box when baseline/_ref is staged (its results race, so
+  * against the stored outputs of the UNMODIFIED reference extension (tests/golden/ref_ext_a.npz; its results race, so
     tolerances + mask IoU instead of exactness, SURVEY.md §8a);
   * the op surface `_C.rasterize_gaussians` (22 arguments -> 11-tuple) and the CLI with its default flags.
 """
@@ -153,49 +153,50 @@ def test_rasterize_gaussians_op_surface(lib):
 
 
 def test_tiles_vs_reference_extension(lib):
-    """Kernels AND oracle against the unmodified reference rasterizer (baseline/_ref, built for sm_100) on this GPU."""
-    from baseline import ref_run
-    if not (ref_run.available() and ref_run.cuda_extension_available()):
-        pytest.skip("baseline/_ref not staged")
+    """Kernels against the unmodified reference rasterizer (built for sm_100, run on a B200): its radii and a fixed
+    pixel sample of every image / depth map, and the per-Gaussian contributions and surface distances accumulated over
+    the cameras, as stored by tests/golden/make_golden.py (ref_ext)."""
+    import os
     import camera_handler as ch
     import gauss_render as gr
     from g2pc import synth
-    from oracle import ref_shim, render_cuda as orc
-    n, res, ncams = 20000, 720, 4
-    sc, cov = _scene(n, 1253)
+    from util import GOLDEN
+    g = np.load(os.path.join(GOLDEN, "ref_ext_a.npz"))
+    n, scene_seed, ncams, res, _, _ = [int(v) for v in g["meta"]]
+    pix = torch.from_numpy(g["pixels"].astype(np.int64)).to(DEV)
+    sc, cov = _scene(n, scene_seed)
     d = scene_to(sc, DEV)
     cams, intr = synth.make_cameras(ncams)
     R = gr.get_renderer("cuda", d["xyz"], d["opacities"].unsqueeze(1), d["colours"], cov.to(DEV),
                         surface_distance_std=2.0, calculate_surface_distance=True)
-    ref = ref_shim.load()
-    with ref_shim.reference_extension():
-        RR = ref.gauss_render.get_renderer("cuda", d["xyz"], d["opacities"].unsqueeze(1), d["colours"], cov.to(DEV),
-                                           surface_distance_std=2.0, calculate_surface_distance=True)
-        worst = 0.0
-        for c2w, k in zip(cams, intr):
-            rs = ch.get_camera("cuda", c2w.to(DEV), k, colour_resolution=res)
-            rrs = ref.camera_handler.get_camera("cuda", c2w.clone().to(DEV), k, colour_resolution=res)
-            img, radii, invd, dep = R(rs)
-            rimg, rradii, rinvd, rdep = RR(rrs)
-            assert int((radii != rradii).sum()) <= max(1, int(3e-4 * n))
-            e = (img - rimg).abs()
-            assert float(e.max()) < 5e-3 and int((e > 2e-4).sum()) <= int(2e-4 * e.numel())
-            worst = max(worst, float(e.max()))
-            ed = (dep - rdep).abs()
-            assert int((ed > 1e-3).sum()) <= int(2e-4 * ed.numel())
+    worst = 0.0
+    for i, (c2w, k) in enumerate(zip(cams, intr)):
+        rs = ch.get_camera("cuda", c2w.to(DEV), k, colour_resolution=res)
+        img, radii, invd, dep = R(rs)
+        assert (rs.image_height, rs.image_width) == tuple(int(v) for v in g["image_hw"])
+        rradii = torch.from_numpy(g["radii"][i].astype(np.int32)).to(DEV)
+        assert int((radii != rradii).sum()) <= max(1, int(3e-4 * n))
+        e = (img.reshape(3, -1)[:, pix] - torch.from_numpy(g["image"][i]).to(DEV)).abs()
+        assert float(e.max()) < 5e-3 and int((e > 2e-4).sum()) <= int(2e-4 * e.numel())
+        worst = max(worst, float(e.max()))
+        ed = (dep.reshape(-1)[pix] - torch.from_numpy(g["depth"][i]).to(DEV)).abs()
+        assert int((ed > 1e-3).sum()) <= int(2e-4 * ed.numel())
     # The reference publishes a Gaussian's per-tile maximum WITHOUT a barrier between the blend loop and the read of the
     # shared maximum (forward.cu:447-456 follows :392-445 directly): a thread whose pixel has finished reads the entry
     # before slower warps have written theirs, so the reference UNDER-reports contributions run-dependently.  The
     # deterministic maximum can therefore only be compared one-sidedly: never below the reference's (up to rounding).
-    km, rm = R.gaussian_max_contribution, RR.gaussian_max_contribution
+    km, rm = R.gaussian_max_contribution, torch.from_numpy(g["max_contribution"]).to(DEV)
     below = int((km < rm - 1e-4).sum())
     off = int(((km - rm).abs() > 1e-4).sum())
     flips = int(((km > 0.05) != (rm > 0.05)).sum())
     lost = int(((rm > 0.05) & ~(km > 0.05)).sum())
-    kt, rt = R.gaussian_total_contribution, RR.gaussian_total_contribution
+    kt, rt = R.gaussian_total_contribution, torch.from_numpy(g["total_contribution"]).to(DEV)
     tbelow = int((kt < rt - 4e-4).sum())
     toff = int(((kt - rt).abs() > 4e-4).sum())
-    ksel, rsel = R.get_gaussians_with_low_surface_distance(), RR.get_gaussians_with_low_surface_distance()
+    # the reference wrapper's selection (get_surface_gaussians_below_distance_threshold) on its stored distances
+    rd = torch.from_numpy(g["min_surface_distance"]).to(DEV)
+    rsel = rd < torch.std_mean(rd[rd < torch.finfo(torch.float).max])[1] * 2.0
+    ksel = R.get_gaussians_with_low_surface_distance()
     iou = float((ksel & rsel).sum()) / max(1.0, float((ksel | rsel).sum()))
     print(f"[vs reference ext] image max diff {worst:.2e}; max contribution: {below} below the reference's, {off}/{n} differ "
           f"(reference under-reports, see comment); total: {tbelow} below, {toff} differ; visibility flips {flips} "
