@@ -41,6 +41,11 @@ SIGNATURES = {
     "g2pc_ppg_workspace_bytes": ([_i64], ctypes.c_int64),
     "g2pc_points_per_gaussian": ([_c_void_p, _c_void_p, _i64, ctypes.c_double, _c_void_p, _c_void_p, _c_void_p, _i64,
                                   _c_void_p], ctypes.c_int),
+    "g2pc_knn_workspace_bytes": ([_i64, _i32], ctypes.c_int64),
+    "g2pc_knn_mean_distance": ([_c_void_p, _i64, _i32, _c_void_p, _c_void_p, _i64, _c_void_p], ctypes.c_int),
+    "g2pc_outlier_workspace_bytes": ([_i64], ctypes.c_int64),
+    "g2pc_outlier_mask": ([_c_void_p, _i64, ctypes.c_double, _c_void_p, _c_void_p, _c_void_p, _i64, _c_void_p],
+                          ctypes.c_int),
     "g2pc_pack_geometry": ([_c_void_p, _c_void_p, _c_void_p, _i64, _c_void_p, _c_void_p], ctypes.c_int),
     "g2pc_preprocess": ([_c_void_p, _c_void_p, _c_void_p, _i32, _i32, _i64, _c_void_p, _c_void_p, _c_void_p, _i32, _u32,
                          _u32, _c_void_p, _c_void_p, _c_void_p, _c_void_p, _c_void_p], ctypes.c_int),
@@ -121,12 +126,13 @@ def load(path=None):
 LAUNCHES = 0      # number of hand-written g2pc kernels launched since the last reset
 TIMING = None     # None, or a dict filled as {entry point name: [(start_event, end_event), ...]}: every launch is
                   # bracketed with CUDA events on the current stream (bench.py)
-# hand-written kernels launched per entry point (default 1); the radix sort inside g2pc_depth_sort is cub's (library)
+# hand-written kernels launched per entry point (default 1); the radix sorts inside g2pc_depth_sort and
+# g2pc_knn_mean_distance are cub's (library)
 _OWN_KERNELS = {"g2pc_multisplit": 5, "g2pc_multisplit_grid": 5, "g2pc_depth_sort": 0, "g2pc_cull_select": 3,
-                "g2pc_points_per_gaussian": 5}
+                "g2pc_points_per_gaussian": 5, "g2pc_knn_mean_distance": 6, "g2pc_outlier_mask": 5}
 _NOT_KERNELS = {"g2pc_version", "g2pc_last_error", "g2pc_sample_emit_chunk_points", "g2pc_multisplit_chunk",
                 "g2pc_multisplit_rows", "g2pc_blend_set_compact", "g2pc_cull_workspace_bytes", "g2pc_ppg_workspace_bytes",
-                "g2pc_depth_sort_workspace_bytes"}
+                "g2pc_depth_sort_workspace_bytes", "g2pc_knn_workspace_bytes", "g2pc_outlier_workspace_bytes"}
 
 
 def call(name, *args):

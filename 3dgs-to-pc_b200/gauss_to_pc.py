@@ -403,7 +403,7 @@ def config_parser(argv=None):
     parser.add_argument("--no_prioritise_visible_gaussians", action="store_true", help="Do not give more points to Gaussians that contribute most")
     parser.add_argument("--visibility_threshold", type=float, default=0.05, help="Minimum contribution each Gaussian must have to be included")
     parser.add_argument("--surface_distance_std", type=float, default=None, help="Cull Gaussians further than X standard deviations from the scene surfaces")
-    parser.add_argument("--clean_pointcloud", action="store_true", help="Remove outliers after generation (requires Open3D)")
+    parser.add_argument("--clean_pointcloud", action="store_true", help="Remove statistical outliers after generation (on the GPU)")
     parser.add_argument("--generate_mesh", action="store_true", help="Also generate a mesh (requires Open3D)")
     parser.add_argument("--poisson_depth", default=10, type=int, help="Depth of the poisson surface reconstruction")
     parser.add_argument("--laplacian_iterations", default=10, type=int, help="Iterations of laplacian mesh smoothing")
@@ -460,13 +460,13 @@ def config_parser(argv=None):
         raise AttributeError("Cannot use masks when no transforms have been provided")
     if args.renderer_type != "cuda" and args.surface_distance_std is not None:
         raise AttributeError("Surface distance calculations only supported in CUDA renderer")
-    if args.clean_pointcloud or args.generate_mesh:
-        # Open3D post-processing is outside this build (SURVEY.md §2 row 15): fail before any loading / rendering
+    if args.generate_mesh:
+        # Open3D meshing is outside this build (SURVEY.md §2 row 15): fail before any loading / rendering
         try:
             import open3d  # noqa: F401
         except ImportError:
-            raise AttributeError("--clean_pointcloud / --generate_mesh need Open3D, which is not installed")
-        raise AttributeError("--clean_pointcloud / --generate_mesh (Open3D post-processing) are not part of this build")
+            raise AttributeError("--generate_mesh needs Open3D, which is not installed")
+        raise AttributeError("--generate_mesh (Open3D meshing) is not part of this build")
 
     return args
 
@@ -504,6 +504,9 @@ def main(argv=None):
                                                                 pointcloud_settings)
 
     if args.clean_pointcloud:
+        if not args.quiet:
+            print("Cleaning Point Cloud")
+            print()
         from mesh_handler import clean_point_cloud
         pts, cols, nrm = clean_point_cloud(total_point_cloud.points, total_point_cloud.colours,
                                            total_point_cloud.normals, device=pointcloud_settings.device)

@@ -154,6 +154,24 @@ int64_t g2pc_ppg_workspace_bytes(int64_t n);
 int g2pc_points_per_gaussian(const float* cov, const float* contrib, int64_t n, double num_points, double* magnitudes,
                              int32_t* ppg, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- point-cloud cleaning: statistical outlier removal (s9_knn.cu) ------------------------------------------------- */
+/* Replaces Open3D's PointCloud.remove_statistical_outlier (mesh_handler.py:89-94, nb_neighbors = k).
+ * avg[i] (n float64) = mean Euclidean distance of point i to its k nearest points of the cloud, itself included (all n
+ * points when n < k); exact kNN over xyz (n,3) f32 through a Morton-ordered bucket tree, distances recomputed in float64.
+ * A point with a non-finite coordinate gets avg = NaN.  1 <= k <= 32, n < 2^31.  workspace: g2pc_knn_workspace_bytes(n,
+ * k), 256-byte aligned (0 for invalid arguments). */
+int64_t g2pc_knn_workspace_bytes(int64_t n, int32_t k);
+int g2pc_knn_mean_distance(const float* xyz, int64_t n, int32_t k, double* avg, void* workspace, int64_t workspace_bytes,
+                           void* stream);
+/* mean = sum of avg over avg > 0, divided by n; std = sqrt(sum over avg > 0 of (avg - mean)^2 / (n - 1)); threshold =
+ * mean + std_ratio * std (fixed-order float64 reductions: bit-identical re-runs).  keep[i] (n uint8) = 0 < avg[i] <
+ * threshold.  stats4 (4 float64, device) = {mean, std, threshold, number of non-finite avg}.  std_ratio > 0.
+ * Compact with g2pc_cull_select(extra_mask = keep) + g2pc_gather_rows.  workspace: g2pc_outlier_workspace_bytes(n),
+ * 8-byte aligned. */
+int64_t g2pc_outlier_workspace_bytes(int64_t n);
+int g2pc_outlier_mask(const double* avg, int64_t n, double std_ratio, uint8_t* keep, double* stats4, void* workspace,
+                      int64_t workspace_bytes, void* stream);
+
 /* ---- S3-S6: colour stage, renderer_type=python semantics (gauss_render.py:101-465) ------------------------------ */
 /* Replaces GaussPythonRenderer.__call__/render (gauss_render.py:266-465) and — as the native op boundary — the role
  * of _C.rasterize_gaussians (rasterize_points.cu:36-145) in the per-camera loop of gauss_to_pc.py:437-454.
