@@ -1,6 +1,9 @@
-// colour_common.cuh — shared pieces of the colour stage (S3-S6): quadtree tables in shared memory, range queries.
+// colour_common.cuh — shared pieces of both colour back-ends (S3-S7): quadtree tables in shared memory, range queries, SH
+// colours, list-table building blocks (block scan, launch-order sort, frame header), async-copy / TMA helpers.
 #pragma once
 #include "common.cuh"
+
+constexpr unsigned FULLM = 0xffffffffu;
 
 #define QT_FLAG_DROPPED 1
 #define QT_FLAG_BIG 2
@@ -28,10 +31,160 @@ __device__ __forceinline__ bool g2pc_frame_skipped(const uint32_t* fail, int fra
     return (uint32_t)(frame + 1) >= *fail;
 }
 
+// Frame header of the list-table kernels (one CTA).  Prologue of a frame that g2pc_frame_skipped: report the poison
+// (the kernel then does nothing).
+__device__ __forceinline__ void report_skipped_frame(const uint32_t* fail, int frame, int32_t* header) {
+    if (threadIdx.x == 0) { header[G2PC_HDR_POISON] = (int32_t)*fail; header[G2PC_HDR_FRAME] = frame; }
+}
+// Epilogue (one thread): the sizes of the frame, the overflow flags, then the failure word — lowered first if the frame
+// did not fit, so the header of a failed frame always names the earliest failure.
+__device__ __forceinline__ void write_frame_header(int32_t* header, uint32_t* fail, int frame, int num_leaves,
+                                                   long long inst_total, int total_pix, int need_deeper, int leaf_over,
+                                                   int cap_over) {
+    header[G2PC_HDR_NUM_LEAVES] = num_leaves;
+    header[G2PC_HDR_TOTAL_INST] = (int32_t)(inst_total & 0xFFFFFFFFll);
+    header[G2PC_HDR_TOTAL_INST_HI] = (int32_t)(inst_total >> 32);
+    header[G2PC_HDR_TOTAL_PIX] = total_pix;
+    header[G2PC_HDR_NEED_DEEPER] = need_deeper;
+    header[G2PC_HDR_LEAF_OVERFLOW] = leaf_over;
+    header[G2PC_HDR_CAP_OVERFLOW] = cap_over;
+    header[G2PC_HDR_FRAME] = frame;
+    if (need_deeper | leaf_over | cap_over) atomicMin(fail, (uint32_t)(frame + 1));
+    const uint32_t f = *(volatile uint32_t*)fail;
+    header[G2PC_HDR_POISON] = f == 0xFFFFFFFFu ? 0 : (int32_t)f;
+}
+
+// block-wide exclusive scan for a CTA of (a multiple of 32, at most 1024) threads; returns the prefix, sets total
+__device__ __forceinline__ int block_scan(int v, int* s_warp, int& total) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(FULLM, inc, o);
+        if (lane >= o) inc += t;
+    }
+    if (lane == 31) s_warp[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+        int w = s_warp[lane];
+        int winc = w;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int t = __shfl_up_sync(FULLM, winc, o);
+            if (lane >= o) winc += t;
+        }
+        s_warp[lane] = winc - w;            // exclusive prefix of warp totals
+        if (lane == 31) s_warp[32] = winc;  // grand total
+    }
+    __syncthreads();
+    const int res = s_warp[warp] + inc - v;
+    total = s_warp[32];
+    __syncthreads();
+    return res;
+}
+
+// Ascending bitonic sort of m keys (a power of two) in shared memory: the heaviest-first launch order of the leaves in
+// both list-table kernels.  NT = threads of the CTA, a compile-time constant (the loop stride unrolls against it).
+template <int NT, typename K>
+__device__ __forceinline__ void bitonic_sort(K* s_sort, int m) {
+    for (int k = 2; k <= m; k <<= 1) {
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int i = threadIdx.x; i < m; i += NT) {
+                const int ixj = i ^ j;
+                if (ixj > i) {
+                    const K a = s_sort[i], b = s_sort[ixj];
+                    const bool up = (i & k) == 0;
+                    if ((a > b) == up) { s_sort[i] = b; s_sort[ixj] = a; }
+                }
+            }
+            __syncthreads();
+        }
+    }
+}
+
+// ---- async copies (sm_90+) --------------------------------------------------------------------------------------------
+__device__ __forceinline__ float ex2f(float x) {
+    float r;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));  // results below FLT_MIN flush to 0
+    return r;
+}
+
+__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
+
+__device__ __forceinline__ void mbar_init(unsigned long long* bar, int count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "WAIT_%=:\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
+        "@p bra DONE_%=;\n"
+        "bra WAIT_%=;\n"
+        "DONE_%=:\n"
+        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
+}
+// one elected thread: arm the barrier with the byte count, then start the 1-D bulk copy global -> shared (TMA engine)
+__device__ __forceinline__ void tma_load_1d(void* dst, const void* src, uint32_t bytes, unsigned long long* bar) {
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // earlier generic-proxy reads of dst are ordered before
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                     smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void cp_async16(void* dst, const void* src) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async4(void* dst, const void* src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+// CTAs of a persistent grid: every SM filled to the kernel's occupancy (per_sm_fallback if the query fails)
+template <typename Kernel>
+inline int resident_ctas(Kernel kernel, int threads, size_t smem, int per_sm_fallback) {
+    int dev = 0, sms = 148, per_sm = per_sm_fallback;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem) != cudaSuccess || per_sm < 1)
+        per_sm = per_sm_fallback;
+    return sms * per_sm;
+}
+
+// SH colour of one channel (gauss_render.py:43-99; + 0.5, clamped at 0 as forward.cu:65-72), d = unit view direction.
+// coef(k) returns coefficient k of the channel; the caller chooses the loads.
+template <typename Coef>
+__device__ __forceinline__ float sh_channel(int deg, float3 d, Coef coef) {
+    const float C0 = 0.28209479177387814f, C1 = 0.4886025119029199f;
+    const float C2[5] = {1.0925484305920792f, -1.0925484305920792f, 0.31539156525252005f, -1.0925484305920792f,
+                         0.5462742152960396f};
+    const float C3[7] = {-0.5900435899266435f, 2.890611442640554f, -0.4570457994644658f, 0.3731763325901154f,
+                         -0.4570457994644658f, 1.445305721320277f, -0.5900435899266435f};
+    const float x = d.x, y = d.y, z = d.z;
+    const float xx = x * x, yy = y * y, zz = z * z, xy = x * y, yz = y * z, xz = x * z;
+    float r = C0 * coef(0);
+    if (deg > 0) {
+        r = r - C1 * y * coef(1) + C1 * z * coef(2) - C1 * x * coef(3);
+        if (deg > 1) {
+            r = r + C2[0] * xy * coef(4) + C2[1] * yz * coef(5) + C2[2] * (2.0f * zz - xx - yy) * coef(6) +
+                C2[3] * xz * coef(7) + C2[4] * (xx - yy) * coef(8);
+            if (deg > 2) {
+                r = r + C3[0] * y * (3.0f * xx - yy) * coef(9) + C3[1] * xy * z * coef(10) +
+                    C3[2] * y * (4.0f * zz - xx - yy) * coef(11) +
+                    C3[3] * z * (2.0f * zz - 3.0f * xx - 3.0f * yy) * coef(12) +
+                    C3[4] * x * (4.0f * zz - xx - yy) * coef(13) + C3[5] * z * (xx - yy) * coef(14) +
+                    C3[6] * x * (xx - 3.0f * yy) * coef(15);
+            }
+        }
+    }
+    return fmaxf(r + 0.5f, 0.0f);
+}
+
 struct QtMeta {
     int32_t num_levels;  // tabulated levels 0..num_levels-1
     int32_t max_gaussians_per_tile;
-    int32_t width, height;
 };
 
 // per-Gaussian projection record: 3 x float4
@@ -42,6 +195,17 @@ struct QtTables {
     const int32_t* xs; const int32_t* xe; const int32_t* xf;
     const int32_t* ys; const int32_t* ye; const int32_t* yf;
 };
+
+// the 6 arrays of n1 ints of the flat table array (g2pc/quadtree.py QuadtreeTables.flat)
+inline QtTables make_tables(const int32_t* tables, int n1) {
+    QtTables t;
+    t.xs = tables; t.xe = tables + n1; t.xf = tables + 2 * n1;
+    t.ys = tables + 3 * n1; t.ye = tables + 4 * n1; t.yf = tables + 5 * n1;
+    return t;
+}
+
+// first 2-D node of level l (levels 0..l-1 hold (4^l - 1) / 3 nodes)
+__device__ __forceinline__ int off2(int l) { return ((1 << (2 * l)) - 1) / 3; }
 
 // copy the 1-D tables (6 arrays of n1 ints) into shared memory; returns pointers into smem
 __device__ __forceinline__ QtTables load_tables(const QtTables g, int n1, int32_t* smem) {
@@ -78,21 +242,6 @@ __device__ __forceinline__ void axis_range(const int32_t* __restrict__ s, const 
     lo = a;
     // hi = last i with s_i < rmax
     a = min(n - 1, max(0, (int)(rmax * inv_step)));
-    while (a >= 0 && !((float)s[a] < rmax)) --a;
-    while (a + 1 < n && (float)s[a + 1] < rmax) ++a;
-    hi = a;
-}
-
-// same query, started from a guess of the answer (lo_guess / hi_guess within a node or two of the exact bounds)
-__device__ __forceinline__ void axis_range_from(const int32_t* __restrict__ s, const int32_t* __restrict__ e, int level,
-                                                float rmin, float rmax, int lo_guess, int hi_guess, int& lo, int& hi) {
-    const int n = 1 << level;
-    if (!(rmax > rmin)) { lo = 1; hi = 0; return; }
-    int a = min(n - 1, max(0, lo_guess));
-    while (a < n && !((float)e[a] > rmin)) ++a;
-    while (a > 0 && (float)e[a - 1] > rmin) --a;
-    lo = a;
-    a = min(n - 1, max(0, hi_guess));
     while (a >= 0 && !((float)s[a] < rmax)) --a;
     while (a + 1 < n && (float)s[a + 1] < rmax) ++a;
     hi = a;

@@ -36,24 +36,14 @@ struct PreParams {
     uint32_t* depth_key;  // bits(-z_view) for Gaussians in front of the camera, 0xFFFFFFFF otherwise
     unsigned long long* val;  // (packed node range at the base level << 32) | Gaussian id
     int32_t nodes_2d;     // histogram entries (0: no shared-memory histogram, global atomics)
-    int32_t hist_off;     // first 2-D node of the shared-memory histogram (= off2(base level))
     uint32_t level_mask;  // bit l: level l has leaf-candidate nodes
     uint32_t clean_mask;  // bit l: level l has no dropped / degenerate node (membership = the looked-up range)
     int32_t base_level;   // lowest set bit of level_mask
 };
 
-__device__ __forceinline__ int off2(int l) { return ((1 << (2 * l)) - 1) / 3; }
-
 __device__ __forceinline__ float3 sh_to_rgb(const float* __restrict__ sh, int stride, int deg, float3 d) {
     // sh: 3 channels x stride coefficients (channel-major).  16-byte loads when the row is 16-byte aligned.
-    const float C0 = 0.28209479177387814f, C1 = 0.4886025119029199f;
-    const float C2[5] = {1.0925484305920792f, -1.0925484305920792f, 0.31539156525252005f, -1.0925484305920792f,
-                         0.5462742152960396f};
-    const float C3[7] = {-0.5900435899266435f, 2.890611442640554f, -0.4570457994644658f, 0.3731763325901154f,
-                         -0.4570457994644658f, 1.445305721320277f, -0.5900435899266435f};
     float out[3];
-    const float x = d.x, y = d.y, z = d.z;
-    const float xx = x * x, yy = y * y, zz = z * z, xy = x * y, yz = y * z, xz = x * z;
     const int ncoef = (deg + 1) * (deg + 1);
     const bool vec = ((stride & 3) == 0) && ((((uintptr_t)sh) & 15) == 0);
 #pragma unroll
@@ -72,21 +62,7 @@ __device__ __forceinline__ float3 sh_to_rgb(const float* __restrict__ sh, int st
 #pragma unroll
             for (int k = 0; k < 16; ++k) if (k < ncoef) s[k] = sh[c * stride + k];
         }
-        float r = C0 * s[0];
-        if (deg > 0) {
-            r = r - C1 * y * s[1] + C1 * z * s[2] - C1 * x * s[3];
-            if (deg > 1) {
-                r = r + C2[0] * xy * s[4] + C2[1] * yz * s[5] + C2[2] * (2.0f * zz - xx - yy) * s[6] +
-                    C2[3] * xz * s[7] + C2[4] * (xx - yy) * s[8];
-                if (deg > 2) {
-                    r = r + C3[0] * y * (3.0f * xx - yy) * s[9] + C3[1] * xy * z * s[10] +
-                        C3[2] * y * (4.0f * zz - xx - yy) * s[11] + C3[3] * z * (2.0f * zz - 3.0f * xx - 3.0f * yy) * s[12] +
-                        C3[4] * x * (4.0f * zz - xx - yy) * s[13] + C3[5] * z * (xx - yy) * s[14] +
-                        C3[6] * x * (xx - 3.0f * yy) * s[15];
-                }
-            }
-        }
-        out[c] = fmaxf(r + 0.5f, 0.0f);
+        out[c] = sh_channel(deg, d, [&](int k) { return s[k]; });
     }
     return make_float3(out[0], out[1], out[2]);
 }
@@ -329,13 +305,6 @@ __global__ void __launch_bounds__(256) pack_geometry_kernel(const float* __restr
     geom[3 * i + 2] = make_float4(c[8], log2f(opacity[i]), 0.0f, 0.0f);
 }
 
-QtTables make_tables(const int32_t* tables, int n1) {
-    QtTables t;
-    t.xs = tables; t.xe = tables + n1; t.xf = tables + 2 * n1;
-    t.ys = tables + 3 * n1; t.ye = tables + 4 * n1; t.yf = tables + 5 * n1;
-    return t;
-}
-
 }  // namespace
 
 extern "C" int g2pc_pack_geometry(const float* xyz, const float* cov, const float* opacity, int64_t n, void* geom,
@@ -369,7 +338,6 @@ extern "C" int g2pc_preprocess(const void* geom, const float* colours, const flo
     p.geom = (const float4*)geom; p.colours = colours; p.shs = shs;
     p.sh_stride = sh_stride; p.sh_degree = sh_degree; p.n = n; p.cam = *cam_host;
     p.meta.num_levels = num_levels; p.meta.max_gaussians_per_tile = 0;
-    p.meta.width = cam_host->width; p.meta.height = cam_host->height;
     p.n1 = (1 << num_levels) - 1;
     p.tab = make_tables(tables, p.n1);
     p.luts = luts;
@@ -379,7 +347,6 @@ extern "C" int g2pc_preprocess(const void* geom, const float* colours, const flo
     p.base_level = __builtin_ctz(level_mask);
     G2PC_CHECK_ARG(p.base_level <= G2PC_RANGE_MAX_LEVEL, "first leaf-candidate level too deep for the packed node range");
     const int nodes_all = ((1 << (2 * num_levels)) - 1) / 3;
-    p.hist_off = 0;
     p.nodes_2d = nodes_all <= 24 * 1024 ? nodes_all : 0;  // histogram in shared memory when it fits (<= 96 KB)
     const size_t lut_bytes = ((size_t)2 * (cam_host->width + cam_host->height) * num_levels * sizeof(uint16_t) + 3) & ~(size_t)3;
     const size_t smem = (size_t)6 * p.n1 * sizeof(int32_t) + (size_t)p.nodes_2d * sizeof(uint32_t) + lut_bytes;
@@ -387,13 +354,9 @@ extern "C" int g2pc_preprocess(const void* geom, const float* colours, const flo
     if (smem > 48 * 1024)
         G2PC_CUDA(cudaFuncSetAttribute(preprocess_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int threads = smem <= 56 * 1024 ? 256 : smem <= 113 * 1024 ? 512 : 1024;
-    int dev = 0, sms = 148, per_sm = 1;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, preprocess_kernel, threads, smem) != cudaSuccess || per_sm < 1)
-        per_sm = 1;
+    const int64_t resident = resident_ctas(preprocess_kernel, threads, smem, 1);
     const int64_t granules = (n + threads - 1) / threads;
-    const unsigned grid = (unsigned)(granules < (int64_t)sms * per_sm ? granules : (int64_t)sms * per_sm);
+    const unsigned grid = (unsigned)(granules < resident ? granules : resident);
     preprocess_kernel<<<grid, threads, smem, (cudaStream_t)stream>>>(p);
     G2PC_CHECK_LAUNCH();
     return G2PC_OK;

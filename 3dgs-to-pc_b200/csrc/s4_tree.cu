@@ -51,37 +51,6 @@ struct TreeParams {
     int32_t nodes_2d;
 };
 
-__device__ __forceinline__ int off2d(int l) { return ((1 << (2 * l)) - 1) / 3; }
-
-// block-wide exclusive scan for TB threads; returns prefix, sets total
-__device__ __forceinline__ int block_scan_1024(int v, int* s_warp, int& total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    int inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int t = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += t;
-    }
-    if (lane == 31) s_warp[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {
-        int w = s_warp[lane];
-        int winc = w;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int t = __shfl_up_sync(0xffffffffu, winc, o);
-            if (lane >= o) winc += t;
-        }
-        s_warp[lane] = winc - w;      // exclusive prefix of warp totals
-        if (lane == 31) s_warp[32] = winc;  // grand total
-    }
-    __syncthreads();
-    const int res = s_warp[warp] + inc - v;
-    total = s_warp[32];
-    __syncthreads();
-    return res;
-}
-
 // key (BFS rank within a level: child rank = 2*xbit + ybit per level, most significant first) -> (ix, iy)
 __device__ __forceinline__ void deinterleave(int key, int level, int& ix, int& iy) {
     ix = 0; iy = 0;
@@ -96,7 +65,7 @@ __global__ void __launch_bounds__(TB) tree_kernel(const TreeParams p) {
     __shared__ int s_flags[2];
     __shared__ unsigned long long s_sort[SORT_CAP];
     if (g2pc_frame_skipped(p.fail, p.frame)) {  // this or an earlier frame failed: report and do nothing
-        if (threadIdx.x == 0) { p.header[G2PC_HDR_POISON] = (int32_t)*p.fail; p.header[G2PC_HDR_FRAME] = p.frame; }
+        report_skipped_frame(p.fail, p.frame, p.header);
         return;
     }
     const int L = p.meta.num_levels;
@@ -106,7 +75,7 @@ __global__ void __launch_bounds__(TB) tree_kernel(const TreeParams p) {
     long long inst_total = 0;
     for (int l = 0; l < L; ++l) {
         const int nn = 1 << (2 * l);
-        const int o1 = (1 << l) - 1, o2 = off2d(l);
+        const int o1 = (1 << l) - 1, o2 = off2(l);
         for (int k0 = 0; k0 < nn; k0 += TB) {
             const int key = k0 + threadIdx.x;
             int is_leaf = 0, node = -1, ix = 0, iy = 0;
@@ -116,7 +85,7 @@ __global__ void __launch_bounds__(TB) tree_kernel(const TreeParams p) {
                 node = o2 + (iy << l) + ix;
                 bool exists = (l == 0);
                 if (l > 0) {
-                    const int pnode = off2d(l - 1) + ((iy >> 1) << (l - 1)) + (ix >> 1);
+                    const int pnode = off2(l - 1) + ((iy >> 1) << (l - 1)) + (ix >> 1);
                     exists = p.node_state[pnode] == NODE_SPLIT;
                 }
                 uint8_t st = NODE_NONE;
@@ -144,7 +113,7 @@ __global__ void __launch_bounds__(TB) tree_kernel(const TreeParams p) {
                 p.node_leaf[node] = nl;
             }
             int tot;
-            const int pre = block_scan_1024(is_leaf, s_warp, tot);
+            const int pre = block_scan(is_leaf, s_warp, tot);
             if (is_leaf) {
                 const int li = leaf_base + pre;
                 if (li < p.max_leaves) {
@@ -176,8 +145,8 @@ __global__ void __launch_bounds__(TB) tree_kernel(const TreeParams p) {
         // every list starts on a 16-byte boundary (the blend stages id chunks with TMA bulk copies): pad to 4 ids
         if (i < nl) { c = (p.leaves[i].inst_count + 3) & ~3; a = p.leaves[i].w * p.leaves[i].h; }
         int tc, ta;
-        const int pc = block_scan_1024(c, s_warp, tc);
-        const int pa = block_scan_1024(a, s_warp, ta);
+        const int pc = block_scan(c, s_warp, tc);
+        const int pa = block_scan(a, s_warp, ta);
         if (i < nl) {
             // 32-bit list offsets: a frame with more than 2^31 instances is reported through the capacity check below
             p.leaves[i].inst_begin = (int32_t)(inst_total + pc);
@@ -202,19 +171,7 @@ __global__ void __launch_bounds__(TB) tree_kernel(const TreeParams p) {
             s_sort[i] = key;
         }
         __syncthreads();
-        for (int k = 2; k <= m; k <<= 1) {
-            for (int j = k >> 1; j > 0; j >>= 1) {
-                for (int i = threadIdx.x; i < m; i += TB) {
-                    const int ixj = i ^ j;
-                    if (ixj > i) {
-                        const unsigned long long a = s_sort[i], b = s_sort[ixj];
-                        const bool up = (i & k) == 0;
-                        if ((a > b) == up) { s_sort[i] = b; s_sort[ixj] = a; }
-                    }
-                }
-                __syncthreads();
-            }
-        }
+        bitonic_sort<TB>(s_sort, m);
         for (int i = threadIdx.x; i < nl; i += TB) p.leaf_order[i] = (int)(s_sort[i] & 0xFFFFull);
     } else {
         for (int i = threadIdx.x; i < nl; i += TB) p.leaf_order[i] = i;
@@ -227,17 +184,7 @@ __global__ void __launch_bounds__(TB) tree_kernel(const TreeParams p) {
                               (long long)p.ms_chunks * (long long)nl > p.matrix_capacity || inst_total > 0x7FFFFFFFll)
                              // (ms_chunks = rows the multisplit needs: chunks + segments, g2pc_multisplit_rows)
                                  ? 1 : 0;
-        p.header[G2PC_HDR_NUM_LEAVES] = leaf_base;
-        p.header[G2PC_HDR_TOTAL_INST] = (int32_t)(inst_total & 0xFFFFFFFFll);
-        p.header[G2PC_HDR_TOTAL_INST_HI] = (int32_t)(inst_total >> 32);
-        p.header[G2PC_HDR_TOTAL_PIX] = pix_base;
-        p.header[G2PC_HDR_NEED_DEEPER] = s_flags[0];
-        p.header[G2PC_HDR_LEAF_OVERFLOW] = s_flags[1];
-        p.header[G2PC_HDR_CAP_OVERFLOW] = cap_over;
-        p.header[G2PC_HDR_FRAME] = p.frame;
-        if (s_flags[0] | s_flags[1] | cap_over) atomicMin(p.fail, (uint32_t)(p.frame + 1));
-        const uint32_t f = *(volatile uint32_t*)p.fail;
-        p.header[G2PC_HDR_POISON] = f == 0xFFFFFFFFu ? 0 : (int32_t)f;
+        write_frame_header(p.header, p.fail, p.frame, leaf_base, inst_total, pix_base, s_flags[0], s_flags[1], cap_over);
     }
 }
 
@@ -330,7 +277,7 @@ __device__ __forceinline__ void for_each_leaf(const MsParams& p, const QtTables&
             if (axlo <= axhi) axis_range(T.ys + ol, T.ye + ol, l, y0, y1, isy0 * (float)(1 << l), aylo, ayhi);
         }
         const bool some = axlo <= axhi && aylo <= ayhi;
-        const int32_t* nl = p.node_leaf + off2d(l);
+        const int32_t* nl = p.node_leaf + off2(l);
         if (((p.clean_mask >> l) & 1u) && l <= G2PC_RANGE_MAX_LEVEL) {
             // no dropped / degenerate node at this level: membership = the range; cooperative walk
             const uint32_t rl = some ? g2pc_pack_range(axlo, axhi, aylo, ayhi) : (uint32_t)G2PC_RANGE_EMPTY;
@@ -363,7 +310,7 @@ __device__ __forceinline__ int32_t* ms_load_common(const MsParams& p, int32_t* s
     }
     int32_t* s_leaf = smem + 6 * p.n1;
     const int nb = 1 << (2 * p.base_level);
-    const int32_t* src = p.node_leaf + off2d(p.base_level);
+    const int32_t* src = p.node_leaf + off2(p.base_level);
     for (int i = threadIdx.x; i < nb; i += blockDim.x) s_leaf[i] = src[i];
     return s_leaf;
 }
@@ -545,10 +492,8 @@ extern "C" int g2pc_build_tree(const int32_t* tables, int32_t num_levels, int32_
     G2PC_CHECK_ARG(frame >= 0 && ms_chunks >= 0, "bad frame / chunk count");
     TreeParams p;
     p.meta.num_levels = num_levels; p.meta.max_gaussians_per_tile = max_gaussians_per_tile;
-    p.meta.width = 0; p.meta.height = 0;
     p.n1 = (1 << num_levels) - 1;
-    p.tab.xs = tables; p.tab.xe = tables + p.n1; p.tab.xf = tables + 2 * p.n1;
-    p.tab.ys = tables + 3 * p.n1; p.tab.ye = tables + 4 * p.n1; p.tab.yf = tables + 5 * p.n1;
+    p.tab = make_tables(tables, p.n1);
     p.node_cnt = node_cnt; p.node_state = node_state; p.node_leaf = node_leaf; p.leaves = leaves;
     p.leaf_order = leaf_order; p.max_leaves = max_leaves;
     p.inst_capacity = inst_capacity; p.pix_capacity = pix_capacity; p.matrix_capacity = matrix_capacity;
@@ -620,10 +565,9 @@ extern "C" int g2pc_multisplit(const uint64_t* val_sorted, int64_t n, const void
     MsParams p;
     p.val_sorted = (const unsigned long long*)val_sorted; p.n = n; p.proj = (const float4*)proj;
     p.width = width; p.height = height;
-    p.meta.num_levels = num_levels; p.meta.max_gaussians_per_tile = 0; p.meta.width = width; p.meta.height = height;
+    p.meta.num_levels = num_levels; p.meta.max_gaussians_per_tile = 0;
     p.n1 = (1 << num_levels) - 1;
-    p.tab.xs = tables; p.tab.xe = tables + p.n1; p.tab.xf = tables + 2 * p.n1;
-    p.tab.ys = tables + 3 * p.n1; p.tab.ye = tables + 4 * p.n1; p.tab.yf = tables + 5 * p.n1;
+    p.tab = make_tables(tables, p.n1);
     p.level_mask = level_mask; p.base_level = __builtin_ctz(level_mask);
     G2PC_CHECK_ARG(p.base_level <= G2PC_RANGE_MAX_LEVEL, "first leaf-candidate level too deep");
     p.node_leaf = node_leaf; p.header = header; p.fail = fail; p.frame = frame; p.leaves = leaves; p.matrix = matrix;
@@ -652,7 +596,7 @@ extern "C" int g2pc_multisplit_grid(const uint64_t* val_sorted, int64_t n, int32
     MsParams p;
     p.val_sorted = (const unsigned long long*)val_sorted; p.n = n; p.proj = nullptr;
     p.width = 0; p.height = 0;
-    p.meta.num_levels = 1; p.meta.max_gaussians_per_tile = 0; p.meta.width = 0; p.meta.height = 0;
+    p.meta.num_levels = 1; p.meta.max_gaussians_per_tile = 0;
     p.n1 = 0;
     p.tab.xs = p.tab.xe = p.tab.xf = p.tab.ys = p.tab.ye = p.tab.yf = nullptr;
     p.level_mask = 1u; p.base_level = 0;

@@ -35,7 +35,6 @@ namespace {
 constexpr int BT = 128;
 constexpr int CH = 128;
 constexpr int SUB = 32;   // Gaussians between two transmittance checks
-constexpr unsigned FULLM = 0xffffffffu;
 
 struct BlendParams {
     const g2pc_leaf_t* leaves;
@@ -57,45 +56,6 @@ struct BlendParams {
     int32_t compact;        // 1: compact warp footprints (blocks), 0: row strips
     unsigned long long* stats;
 };
-
-__device__ __forceinline__ float ex2f(float x) {
-    float r;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));  // results below FLT_MIN flush to 0 (see header comment)
-    return r;
-}
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-// one elected thread: arm the barrier with the byte count, then start the 1-D bulk copy global -> shared (TMA engine)
-__device__ __forceinline__ void tma_load_1d(void* dst, const void* src, uint32_t bytes, unsigned long long* bar) {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // earlier generic-proxy reads of dst are ordered before
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void cp_async16(void* dst, const void* src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async4(void* dst, const void* src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 __global__ void __launch_bounds__(BT, 8) blend_kernel(const BlendParams p) {
     __shared__ __align__(16) float4 s_q0[2][CH];
@@ -382,14 +342,7 @@ extern "C" int g2pc_blend(const g2pc_leaf_t* leaves, const int32_t* leaf_order, 
     p.work_counter = work_counters;
     p.stats = (unsigned long long*)stats;
     static int resident = 0;  // persistent grid: every SM filled to the kernel's occupancy (device constant)
-    if (resident == 0) {
-        int dev = 0, sms = 148, per_sm = 8;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, blend_kernel, BT, 0) != cudaSuccess || per_sm < 1)
-            per_sm = 8;
-        resident = sms * per_sm;
-    }
+    if (resident == 0) resident = resident_ctas(blend_kernel, BT, 0, 8);
     blend_kernel<<<(unsigned)resident, BT, 0, (cudaStream_t)stream>>>(p);
     G2PC_CHECK_LAUNCH();
     return G2PC_OK;

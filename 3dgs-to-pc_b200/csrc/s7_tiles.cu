@@ -25,7 +25,6 @@
 namespace {
 
 constexpr int TILE = 16;
-constexpr unsigned FULLM = 0xffffffffu;
 
 struct TilePreParams {
     const float4* geom;    // packed geometry (g2pc_pack_geometry)
@@ -45,33 +44,10 @@ struct TilePreParams {
 };
 
 __device__ __forceinline__ float3 sh_eval(const float* __restrict__ sh, int stride, int layout, int deg, float3 d) {
-    const float C0 = 0.28209479177387814f, C1 = 0.4886025119029199f;
-    const float C2[5] = {1.0925484305920792f, -1.0925484305920792f, 0.31539156525252005f, -1.0925484305920792f,
-                         0.5462742152960396f};
-    const float C3[7] = {-0.5900435899266435f, 2.890611442640554f, -0.4570457994644658f, 0.3731763325901154f,
-                         -0.4570457994644658f, 1.445305721320277f, -0.5900435899266435f};
-    const float x = d.x, y = d.y, z = d.z;
-    const float xx = x * x, yy = y * y, zz = z * z, xy = x * y, yz = y * z, xz = x * z;
     float out[3];
 #pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        auto S = [&](int k) { return layout == 0 ? __ldg(sh + c * stride + k) : __ldg(sh + 3 * k + c); };
-        float r = C0 * S(0);
-        if (deg > 0) {
-            r = r - C1 * y * S(1) + C1 * z * S(2) - C1 * x * S(3);
-            if (deg > 1) {
-                r = r + C2[0] * xy * S(4) + C2[1] * yz * S(5) + C2[2] * (2.0f * zz - xx - yy) * S(6) + C2[3] * xz * S(7) +
-                    C2[4] * (xx - yy) * S(8);
-                if (deg > 2) {
-                    r = r + C3[0] * y * (3.0f * xx - yy) * S(9) + C3[1] * xy * z * S(10) +
-                        C3[2] * y * (4.0f * zz - xx - yy) * S(11) + C3[3] * z * (2.0f * zz - 3.0f * xx - 3.0f * yy) * S(12) +
-                        C3[4] * x * (4.0f * zz - xx - yy) * S(13) + C3[5] * z * (xx - yy) * S(14) +
-                        C3[6] * x * (xx - 3.0f * yy) * S(15);
-                }
-            }
-        }
-        out[c] = fmaxf(r + 0.5f, 0.0f);
-    }
+    for (int c = 0; c < 3; ++c)
+        out[c] = sh_channel(deg, d, [&](int k) { return layout == 0 ? __ldg(sh + c * stride + k) : __ldg(sh + 3 * k + c); });
     return make_float3(out[0], out[1], out[2]);
 }
 
@@ -196,34 +172,6 @@ __global__ void __launch_bounds__(256) preprocess_tiles_kernel(const TilePrePara
 constexpr int TB = 1024;
 constexpr int SORT_CAP = 8192;
 
-__device__ __forceinline__ int block_scan(int v, int* s_warp, int& total) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    int inc = v;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int t = __shfl_up_sync(FULLM, inc, o);
-        if (lane >= o) inc += t;
-    }
-    if (lane == 31) s_warp[warp] = inc;
-    __syncthreads();
-    if (warp == 0) {
-        int w = s_warp[lane];
-        int winc = w;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int t = __shfl_up_sync(FULLM, winc, o);
-            if (lane >= o) winc += t;
-        }
-        s_warp[lane] = winc - w;
-        if (lane == 31) s_warp[32] = winc;
-    }
-    __syncthreads();
-    const int res = s_warp[warp] + inc - v;
-    total = s_warp[32];
-    __syncthreads();
-    return res;
-}
-
 struct TileTreeParams {
     uint32_t* node_cnt;
     g2pc_leaf_t* leaves;
@@ -240,7 +188,7 @@ __global__ void __launch_bounds__(TB) tile_tree_kernel(const TileTreeParams p) {
     __shared__ int s_warp[33];
     __shared__ uint32_t s_sort[SORT_CAP];  // (2^19 - 1 - min(count, 2^19 - 1)) << 13 | tile
     if (g2pc_frame_skipped(p.fail, p.frame)) {
-        if (threadIdx.x == 0) { p.header[G2PC_HDR_POISON] = (int32_t)*p.fail; p.header[G2PC_HDR_FRAME] = p.frame; }
+        report_skipped_frame(p.fail, p.frame, p.header);
         return;
     }
     const int nt = p.gx * p.gy;  // (gx, gy = super-tile grid here)
@@ -275,19 +223,7 @@ __global__ void __launch_bounds__(TB) tile_tree_kernel(const TileTreeParams p) {
             s_sort[i] = key;
         }
         __syncthreads();
-        for (int k = 2; k <= m; k <<= 1) {
-            for (int j = k >> 1; j > 0; j >>= 1) {
-                for (int i = threadIdx.x; i < m; i += TB) {
-                    const int ixj = i ^ j;
-                    if (ixj > i) {
-                        const uint32_t a = s_sort[i], b = s_sort[ixj];
-                        const bool up = (i & k) == 0;
-                        if ((a > b) == up) { s_sort[i] = b; s_sort[ixj] = a; }
-                    }
-                }
-                __syncthreads();
-            }
-        }
+        bitonic_sort<TB>(s_sort, m);
         for (int i = threadIdx.x; i < nl; i += TB) p.leaf_order[i] = (int)(s_sort[i] & 0x1FFFu);
     } else {
         for (int i = threadIdx.x; i < nl; i += TB) p.leaf_order[i] = i;
@@ -299,17 +235,7 @@ __global__ void __launch_bounds__(TB) tile_tree_kernel(const TileTreeParams p) {
         const int leaf_over = nt > p.max_leaves ? 1 : 0;
         const int cap_over = (inst_total > p.inst_capacity || (long long)p.ms_rows * (long long)nl > p.matrix_capacity ||
                               inst_total > 0x7FFFFFFFll) ? 1 : 0;
-        p.header[G2PC_HDR_NUM_LEAVES] = nt;
-        p.header[G2PC_HDR_TOTAL_INST] = (int32_t)(inst_total & 0xFFFFFFFFll);
-        p.header[G2PC_HDR_TOTAL_INST_HI] = (int32_t)(inst_total >> 32);
-        p.header[G2PC_HDR_TOTAL_PIX] = p.W * p.H;
-        p.header[G2PC_HDR_NEED_DEEPER] = 0;
-        p.header[G2PC_HDR_LEAF_OVERFLOW] = leaf_over;
-        p.header[G2PC_HDR_CAP_OVERFLOW] = cap_over;
-        p.header[G2PC_HDR_FRAME] = p.frame;
-        if (leaf_over | cap_over) atomicMin(p.fail, (uint32_t)(p.frame + 1));
-        const uint32_t f = *(volatile uint32_t*)p.fail;
-        p.header[G2PC_HDR_POISON] = f == 0xFFFFFFFFu ? 0 : (int32_t)f;
+        write_frame_header(p.header, p.fail, p.frame, nt, inst_total, p.W * p.H, 0, leaf_over, cap_over);
     }
 }
 
@@ -343,39 +269,6 @@ struct TileBlendParams {
     unsigned long long* stats;
 };
 
-__device__ __forceinline__ float ex2a(float x) {
-    float r;
-    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-    return r;
-}
-__device__ __forceinline__ uint32_t s_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mb_init(unsigned long long* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mb_wait(unsigned long long* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(s_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void tma_1d(void* dst, const void* src, uint32_t bytes, unsigned long long* bar) {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_u32(bar)), "r"(bytes) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                     s_u32(dst)), "l"(src), "r"(bytes), "r"(s_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void cpa16(void* dst, const void* src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s_u32(dst)), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cpa_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cpa_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
 __device__ __forceinline__ void pair_sync(int tile) {  // the two warps of one tile (static ids: a register id makes
     switch (tile) {                                     // ptxas reserve all 16 barriers and caps the CTAs per SM)
         case 0: asm volatile("bar.sync 1, 64;" ::: "memory"); break;
@@ -404,7 +297,7 @@ __global__ void __launch_bounds__(TBT, SURF ? 3 : 4) blend_tiles_kernel(const Ti
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int tile = tid >> 6, tt = tid & 63;  // tile of the super-tile, thread of the tile
     if (tid == 0) {
-        mb_init(&s_bar[0], 1); mb_init(&s_bar[1], 1); mb_init(&s_bar[2], 1);
+        mbar_init(&s_bar[0], 1); mbar_init(&s_bar[1], 1); mbar_init(&s_bar[2], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     for (int w = 0; w < TBT / 32; ++w)
@@ -449,22 +342,22 @@ __global__ void __launch_bounds__(TBT, SURF ? 3 : 4) blend_tiles_kernel(const Ti
 
     auto issue_ids = [&](int c) {
         const int nl = min(TCH, cnt - c * TCH);
-        tma_1d(&s_gid[c % 3][0], list + (int64_t)c * TCH, (uint32_t)(((nl + 3) & ~3) * 4), &s_bar[c % 3]);
+        tma_load_1d(&s_gid[c % 3][0], list + (int64_t)c * TCH, (uint32_t)(((nl + 3) & ~3) * 4), &s_bar[c % 3]);
     };
     auto wait_ids = [&](int c) {
         const int s = c % 3;
-        mb_wait(&s_bar[s], (phase_bits >> s) & 1u);
+        mbar_wait(&s_bar[s], (phase_bits >> s) & 1u);
         phase_bits ^= 1u << s;
     };
     auto issue_records = [&](int c) {
         const int nl = min(TCH, cnt - c * TCH);
         if (tid < nl) {
             const float4* rec = p.proj + 3 * (int64_t)s_gid[c % 3][tid];
-            cpa16(&s_q0[c & 1][tid], rec);
-            cpa16(&s_q1[c & 1][tid], rec + 1);
-            cpa16(&s_q2[c & 1][tid], rec + 2);
+            cp_async16(&s_q0[c & 1][tid], rec);
+            cp_async16(&s_q1[c & 1][tid], rec + 1);
+            cp_async16(&s_q2[c & 1][tid], rec + 2);
         }
-        cpa_commit();
+        cp_async_commit();
     };
     // end of a round of the tile's list (forward.cu:460-477): distance of every entry of the round to the nearest running
     // expected depth among the tile's 256 threads.  Sort the values once, then binary-search per entry.  Both warps of
@@ -511,10 +404,10 @@ __global__ void __launch_bounds__(TBT, SURF ? 3 : 4) blend_tiles_kernel(const Ti
         const int nload = min(TCH, cnt - c * TCH);
         const bool more = (c + 1 < nchunks);
         if (more) { wait_ids(c + 1); issue_records(c + 1); }
-        if (more) cpa_wait<1>(); else cpa_wait<0>();
+        if (more) cp_async_wait<1>(); else cp_async_wait<0>();
         const bool all_left = __syncthreads_and((SURF ? tile_left : (tile_left || warp_done)) ? 1 : 0);
         if (all_left) {
-            if (more) cpa_wait<0>();
+            if (more) cp_async_wait<0>();
             break;
         }
         if (tid == 0 && c + 2 < nchunks) issue_ids(c + 2);
@@ -559,7 +452,7 @@ __global__ void __launch_bounds__(TBT, SURF ? 3 : 4) blend_tiles_kernel(const Ti
                     for (int i = 0; i < 4; ++i) {
                         const float dx = px[i] - q0.x;
                         const float pw = fmaf(dx, fmaf(dx, q0.z, Bq), Cq);  // = power * log2(e)
-                        const float alpha = fminf(0.99f, ex2a(pw + q1.y));
+                        const float alpha = fminf(0.99f, ex2f(pw + q1.y));
                         // power > 0 -> skip; alpha < 1/255 -> skip (forward.cu:404,412)
                         const bool keep = !(pw > 0.0f) && !(alpha < (1.0f / 255.0f));
                         const float cand = T[i] * alpha;
@@ -743,18 +636,11 @@ extern "C" int g2pc_tiles_blend(const g2pc_leaf_t* leaves, const int32_t* leaf_o
     p.W = width; p.H = height;
     for (int i = 0; i < 3; ++i) p.bg[i] = background3_host[i];
     p.work_counter = work_counters; p.stats = (unsigned long long*)stats;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     cudaStream_t st = (cudaStream_t)stream;
-    int per_sm = 3;
-    if (cam_dist) {
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, blend_tiles_kernel<true>, TBT, 0) != cudaSuccess || per_sm < 1) per_sm = 3;
-        blend_tiles_kernel<true><<<(unsigned)(sms * per_sm), TBT, 0, st>>>(p);
-    } else {
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, blend_tiles_kernel<false>, TBT, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
-        blend_tiles_kernel<false><<<(unsigned)(sms * per_sm), TBT, 0, st>>>(p);
-    }
+    if (cam_dist)
+        blend_tiles_kernel<true><<<(unsigned)resident_ctas(blend_tiles_kernel<true>, TBT, 0, 3), TBT, 0, st>>>(p);
+    else
+        blend_tiles_kernel<false><<<(unsigned)resident_ctas(blend_tiles_kernel<false>, TBT, 0, 4), TBT, 0, st>>>(p);
     G2PC_CHECK_LAUNCH();
     return G2PC_OK;
 }

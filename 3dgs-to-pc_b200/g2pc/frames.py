@@ -23,12 +23,12 @@ _HDR_POOLS = {}  # device -> free pinned frame headers (cudaHostAlloc is slow: n
 
 
 class FrameQueue:
-    """Mixin.  The owner provides: self.device, self._ensure_buffers(camera, slot) (allocate / grow the slot's scratch on
-    the current stream), self._enqueue_front(camera, frame, slot) -> device header tensor,
-    self._enqueue_back(camera, frame, camera_index, slot), self._fix(header_list), self._confirm(header_list) and
-    self._reset_counts() (zero the per-slot tile counters after a failure)."""
+    """Mixin.  The owner provides: self.device, self.lib, self._ensure_buffers(camera, slot) (allocate / grow the slot's
+    scratch on the current stream), self._enqueue_front(camera, frame, slot) -> device header tensor,
+    self._enqueue_back(camera, frame, camera_index, slot), self._fix(header_list) and self._confirm(header_list).
+    self._tables maps a resolution to its tables, each with a "slots" list of per-slot dicts holding "node_cnt"."""
 
-    def _init_frames(self):
+    def _init_frames(self, n):
         self._frame = 0
         self._pending = []   # (frame, camera, camera_index, pinned header, end-of-frame event)
         self._hdr_pool = _HDR_POOLS.setdefault(str(self.device), [])  # pinned headers are shared by all renderers
@@ -38,6 +38,53 @@ class FrameQueue:
         self._streams = [torch.cuda.Stream(device=self.device) for _ in range(self.num_slots)]
         self._fail = torch.full((1,), -1, dtype=torch.int32, device=self.device)  # 0xFFFFFFFF: no frame has failed
         self._prev_done = None
+        # per-frame scratch: one set per slot (frames alternate between the slots)
+        dev = self.device
+        m = max(n, 1)
+        nbytes = self.lib.g2pc_depth_sort_workspace_bytes(m)
+        self._slots = [dict(proj=torch.empty((m, 12), dtype=torch.float32, device=dev),
+                            depth_key=torch.empty((m,), dtype=torch.int32, device=dev),
+                            val=torch.empty((m,), dtype=torch.int64, device=dev),
+                            val_sorted=torch.empty((m,), dtype=torch.int64, device=dev),
+                            depth_ws=torch.empty((max(int(nbytes), 1),), dtype=torch.uint8, device=dev),
+                            hdr=torch.zeros((capi.HDR_WORDS,), dtype=torch.int32, device=dev),
+                            work=torch.zeros((capi.WORK_COUNTERS,), dtype=torch.int32, device=dev),
+                            inst_gid=None, matrix=None) for _ in range(self.num_slots)]
+        self._cam_best = torch.zeros((m,), dtype=torch.int64, device=dev)
+        self._stats = torch.zeros((capi.STAT_WORDS,), dtype=torch.int64, device=dev)
+        self._inst_cap = max(8 * n, 1 << 16)  # (Gaussian, list) instances; grown when a frame overflows
+        self._tables = {}
+        self._last_slot = 0
+        self.last_stats = {}
+
+    def _grow_lists(self, sl, lists, matrix_rows):
+        """Grow the slot's list buffer (inst_gid) to _inst_cap instances in `lists` lists and its multisplit matrix to
+        matrix_rows x lists."""
+        need = self._inst_cap + 4 * lists + 64  # lists are padded to 16 bytes; slack for the last TMA unit
+        if sl["inst_gid"] is None or sl["inst_gid"].numel() < need:
+            sl["inst_gid"] = torch.empty((need,), dtype=torch.int32, device=self.device)
+        mneed = matrix_rows * lists
+        if sl["matrix"] is None or sl["matrix"].numel() < mneed:
+            sl["matrix"] = torch.empty((max(mneed, 1),), dtype=torch.int32, device=self.device)
+
+    def _grow_inst_cap(self, h):
+        """The frame of header h had more (Gaussian, tile) instances than _inst_cap: grow it."""
+        total = h[capi.HDR_TOTAL_INST] + (h[capi.HDR_TOTAL_INST_HI] << 32)
+        if total > 0x7FFFFFFF:
+            raise capi.G2pcError(f"{total} (Gaussian, tile) instances in one camera: more than 2^31 - 1")
+        self._inst_cap = max(self._inst_cap, int(1.25 * total) + 1024)
+
+    def _reset_counts(self):
+        """Zero the per-slot tile counters (a failed frame left them half counted)."""
+        for t in self._tables.values():
+            for ts in t["slots"]:
+                ts["node_cnt"].zero_()
+
+    def executed_pairs(self):
+        """(pixel, Gaussian) pairs the blend evaluated since construction: 32 threads x 4 pixels per warp and Gaussian
+        (device counter)."""
+        self.flush()
+        return int(self._stats[capi.STAT_WARP_GAUSSIANS].item()) * 128
 
     def _launch(self, frame, camera, camera_index):
         slot = frame % self.num_slots

@@ -130,28 +130,14 @@ class GaussianRasterizer(FrameQueue):
         if shs is not None:
             self._shs_f32 = shs.to(torch.float32).contiguous()
             self._sh_stride = int(self._shs_f32.shape[2] if self._sh_layout == 0 else self._shs_f32.shape[1])
-        self._init_frames()
+        self._init_frames(n)
         m = max(n, 1)
-        nbytes = self.lib.g2pc_depth_sort_workspace_bytes(m)
-        self._slots = [dict(proj=torch.empty((m, 12), dtype=torch.float32, device=dev),
-                            depth_key=torch.empty((m,), dtype=torch.int32, device=dev),
-                            val=torch.empty((m,), dtype=torch.int64, device=dev),
-                            val_sorted=torch.empty((m,), dtype=torch.int64, device=dev),
-                            depth_ws=torch.empty((max(int(nbytes), 1),), dtype=torch.uint8, device=dev),
-                            hdr=torch.zeros((capi.HDR_WORDS,), dtype=torch.int32, device=dev),
-                            work=torch.zeros((capi.WORK_COUNTERS,), dtype=torch.int32, device=dev),
-                            radii=torch.zeros((m,), dtype=torch.int32, device=dev),
-                            inst_gid=None, matrix=None) for _ in range(self.num_slots)]
-        self._cam_best = torch.zeros((m,), dtype=torch.int64, device=dev)
+        for sl in self._slots:
+            sl["radii"] = torch.zeros((m,), dtype=torch.int32, device=dev)
         self._cam_dist = None
         if calculate_surface_distance:
             self._cam_dist = torch.empty((m,), dtype=torch.int32, device=dev)
             capi.call("g2pc_fill_u32", capi.ptr(self._cam_dist), FLT_MAX_BITS, m, capi.stream_ptr(dev))
-        self._stats = torch.zeros((capi.STAT_WORDS,), dtype=torch.int64, device=dev)
-        self._inst_cap = max(8 * n, 1 << 16)  # 32x32 super-tiles: a splat of radius ~15 px touches 4-9 of them
-        self._res = {}
-        self._last_slot = 0
-        self.last_stats = {}
 
     # ---- nn.Module-like call surface -----------------------------------------------------------------------------------
     def __call__(self, raster_settings, **kw):
@@ -170,7 +156,7 @@ class GaussianRasterizer(FrameQueue):
         self._packed, self._scale_modifier = True, scale_modifier
 
     def _res_tables(self, W, H):
-        t = self._res.get((W, H))
+        t = self._tables.get((W, H))
         if t is None:
             dev = self.device
             # the depth-ordered lists are built per super-tile of 2x2 tiles (csrc/s7_tiles.cu)
@@ -187,17 +173,8 @@ class GaussianRasterizer(FrameQueue):
                      colour=torch.zeros((3, H, W), dtype=torch.float32, device=dev),
                      depth=torch.zeros((1, H, W), dtype=torch.float32, device=dev),
                      invdepth=torch.zeros((1, H, W), dtype=torch.float32, device=dev))
-            self._res[(W, H)] = t
+            self._tables[(W, H)] = t
         return t
-
-    def _buffers(self, t, sl):
-        dev = self.device
-        need = self._inst_cap + 4 * t["ntiles"] + 64
-        if sl["inst_gid"] is None or sl["inst_gid"].numel() < need:
-            sl["inst_gid"] = torch.empty((need,), dtype=torch.int32, device=dev)
-        mneed = t["rows"] * t["ntiles"]
-        if sl["matrix"] is None or sl["matrix"].numel() < mneed:
-            sl["matrix"] = torch.empty((max(mneed, 1),), dtype=torch.int32, device=dev)
 
     def _mask_of(self, rs, W, H):
         mask = rs.mask
@@ -212,7 +189,7 @@ class GaussianRasterizer(FrameQueue):
     def _ensure_buffers(self, rs, slot):
         self._pack(float(rs.scale_modifier))
         t = self._res_tables(int(rs.image_width), int(rs.image_height))
-        self._buffers(t, self._slots[slot])
+        self._grow_lists(self._slots[slot], t["ntiles"], t["rows"])
         # (kept per slot: the tensor must outlive the frame's kernels, the slot is reused only after they have run)
         self._slots[slot]["mask"] = self._mask_of(rs, int(rs.image_width), int(rs.image_height))
 
@@ -277,22 +254,9 @@ class GaussianRasterizer(FrameQueue):
 
     def _fix(self, h):
         if h[capi.HDR_CAP_OVERFLOW]:
-            total = h[capi.HDR_TOTAL_INST] + (h[capi.HDR_TOTAL_INST_HI] << 32)
-            if total > 0x7FFFFFFF:
-                raise capi.G2pcError(f"{total} (Gaussian, tile) instances in one camera: more than 2^31 - 1")
-            self._inst_cap = max(self._inst_cap, int(1.25 * total) + 1024)
+            self._grow_inst_cap(h)
         else:
             raise capi.G2pcError("failed frame header without a recoverable cause")
-
-    def _reset_counts(self):
-        for t in self._res.values():
-            for ts in t["slots"]:
-                ts["node_cnt"].zero_()
-
-    def executed_pairs(self):
-        """(pixel, Gaussian) pairs the blend evaluated since construction: 64 threads x 4 pixels per tile, 2 warps."""
-        self.flush()
-        return int(self._stats[capi.STAT_WARP_GAUSSIANS].item()) * 128
 
     # ---- accumulator updates kept for API parity (the kernels fuse them) -------------------------------------------------
     def update_max_contributions(self, new_gauss_contributions, new_gauss_colours):

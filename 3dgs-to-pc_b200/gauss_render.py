@@ -81,7 +81,6 @@ class GaussPythonRenderer(FrameQueue):
         self.compose_image = True
         self.async_mode = False
         self.first_frame = None  # optional (n) int32: index of the camera that raised each maximum (g2pc/dist.py)
-        self._tables = {}
         self._extra_levels = 0
         self._n = n
         st = capi.stream_ptr(dev)
@@ -89,24 +88,8 @@ class GaussPythonRenderer(FrameQueue):
         self._geom = torch.empty((max(n, 1), 12), dtype=torch.float32, device=dev)
         capi.call("g2pc_pack_geometry", capi.ptr(self.means3D), capi.ptr(self.cov3d), capi.ptr(self.opacity), n,
                   capi.ptr(self._geom), st)
-        self._init_frames()
-        # per-frame scratch: one set per slot (frames alternate between the slots)
-        m = max(n, 1)
-        nbytes = self.lib.g2pc_depth_sort_workspace_bytes(m)
-        self._slots = [dict(proj=torch.empty((m, 12), dtype=torch.float32, device=dev),
-                            depth_key=torch.empty((m,), dtype=torch.int32, device=dev),
-                            val=torch.empty((m,), dtype=torch.int64, device=dev),
-                            val_sorted=torch.empty((m,), dtype=torch.int64, device=dev),
-                            depth_ws=torch.empty((max(int(nbytes), 1),), dtype=torch.uint8, device=dev),
-                            hdr=torch.zeros((capi.HDR_WORDS,), dtype=torch.int32, device=dev),
-                            work=torch.zeros((capi.WORK_COUNTERS,), dtype=torch.int32, device=dev),
-                            inst_gid=None, matrix=None) for _ in range(self.num_slots)]
-        self._cam_best = torch.zeros((m,), dtype=torch.int64, device=dev)
-        self._stats = torch.zeros((capi.STAT_WORDS,), dtype=torch.int64, device=dev)
+        self._init_frames(n)
         self._leaf_colour = None
-        self._inst_cap = max(8 * n, 1 << 16)
-        self._last_slot = 0
-        self.last_stats = {}
 
     # ---- getters (gauss_render.py:237-264) -----------------------------------------------------------------
     def get_gaussian_colours(self):
@@ -128,11 +111,6 @@ class GaussPythonRenderer(FrameQueue):
         # the python back-end of the reference reports the MAX contribution here (gauss_render.py:261-264)
         self.flush()
         return self.gaussian_max_contribution
-
-    def executed_pairs(self):
-        """(pixel, Gaussian) pairs the blend kernel evaluated since construction (device counter)."""
-        self.flush()
-        return int(self._stats[capi.STAT_WARP_GAUSSIANS].item()) * 128
 
     # ---- per-resolution tables ---------------------------------------------------------------------------------
     def _get_tables(self, W, H):
@@ -199,21 +177,12 @@ class GaussPythonRenderer(FrameQueue):
         c.height = camera.image_height
         return c
 
-    def _buffers(self, t, sl):
-        """(Re)allocate the slot's frame buffers for the current capacities."""
-        dev = self.device
-        need = self._inst_cap + 4 * t["leaf_cap"] + 64  # lists are padded to 16 bytes; slack for the last TMA unit
-        if sl["inst_gid"] is None or sl["inst_gid"].numel() < need:
-            sl["inst_gid"] = torch.empty((need,), dtype=torch.int32, device=dev)
-        if self._leaf_colour is None or self._leaf_colour.numel() < 3 * t["pix_cap"]:
-            self._leaf_colour = torch.empty((3 * t["pix_cap"],), dtype=torch.float32, device=dev)
-        mneed = t["chunks"] * t["leaf_cap"]
-        if sl["matrix"] is None or sl["matrix"].numel() < mneed:
-            sl["matrix"] = torch.empty((max(mneed, 1),), dtype=torch.int32, device=dev)
-
     def _ensure_buffers(self, camera, slot):
+        """(Re)allocate the slot's frame buffers for the current capacities."""
         t = self._get_tables(int(camera.image_width), int(camera.image_height))
-        self._buffers(t, self._slots[slot])
+        self._grow_lists(self._slots[slot], t["leaf_cap"], t["chunks"])
+        if self._leaf_colour is None or self._leaf_colour.numel() < 3 * t["pix_cap"]:
+            self._leaf_colour = torch.empty((3 * t["pix_cap"],), dtype=torch.float32, device=self.device)
 
     def _enqueue_front(self, camera, frame, slot):
         """Projection, depth sort, tile table and per-tile lists of one camera, asynchronously on the current stream."""
@@ -299,18 +268,10 @@ class GaussPythonRenderer(FrameQueue):
                 raise capi.G2pcError("leaf table overflow")
             self._set_leaf_cap(t, max(2 * t["leaf_cap"], int(1.25 * h[capi.HDR_NUM_LEAVES])))
         elif h[capi.HDR_CAP_OVERFLOW]:
-            total = h[capi.HDR_TOTAL_INST] + (h[capi.HDR_TOTAL_INST_HI] << 32)
-            if total > 0x7FFFFFFF:
-                raise capi.G2pcError(f"{total} (Gaussian, tile) instances in one camera: more than 2^31 - 1")
-            self._inst_cap = max(self._inst_cap, int(1.25 * total) + 1024)
+            self._grow_inst_cap(h)
             t["pix_cap"] = max(t["pix_cap"], int(1.25 * h[capi.HDR_TOTAL_PIX]) + 1024)
         else:
             raise capi.G2pcError("poisoned frame header without a cause")
-
-    def _reset_counts(self):
-        for tt in self._tables.values():
-            for ts in tt["slots"]:
-                ts["node_cnt"].zero_()
 
     # ---- introspection for the parity tests ---------------------------------------------------------------------
     def debug_last_camera(self):
